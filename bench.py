@@ -35,6 +35,10 @@ import numpy as np
 REPO = os.path.dirname(os.path.abspath(__file__))
 if REPO not in sys.path:
     sys.path.insert(0, REPO)
+# The tree the benchmark runs from may be read-only: no bytecode caches in it, from this process or the ones it starts.
+# Whatever else it builds goes to a temporary directory.
+sys.dont_write_bytecode = True
+os.environ["PYTHONDONTWRITEBYTECODE"] = "1"
 
 METRIC = "simulated events/sec (100k-job trace, 4x32x8 cluster)"
 # --config: c1 = the BASELINE metric's configuration (default); c5 = BASELINE configs[4]: 16x64x8 cluster, 1M-job trace
@@ -139,6 +143,64 @@ def run_to_done(eng, rows_cap, totals=None):
                 t[0] += int(w.ev_rows); t[1] += int(w.q_rows)
         if all(eng.stats(s).done for s in range(eng.nsims)):
             return
+
+
+DUMP_SEED = 0
+DUMP_REPLICAS, DUMP_JOBS, DUMP_ROWS = 3, 100000, 4096      # 43 MB on the c1 workload
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(eng, out_dir):
+    """Write what the last timed step computed, as the engine's caller receives it (gs_stats, gs_window, gs_fetch_rows,
+    gs_fetch_jobs, gs_fetch_spans), to out_dir/<name>.npy: 2-D float64 tables whose first column is the replica.
+    The samples are drawn with a fixed seed, so two builds run with the same arguments write comparable files.
+
+      replica_stats : every replica: ticks, events, finished, started, placement_evals, done,
+                      ev_rows, q_rows, node_events, spans_used, admitted
+      jobs          : DUMP_REPLICAS sampled replicas x up to DUMP_JOBS sampled jobs: job, start, end, jct, preempt, duration
+      finish_order  : the same replicas, up to DUMP_JOBS sampled positions: position, job
+      spans         : the placement spans of the sampled jobs: job, node, ntasks, devmask
+      rows          : the same replicas, up to DUMP_ROWS sampled statistics rows (the last one always): the gs_tick_row fields
+    """
+    from gpuschedule_b200.log_manager import ROW_DTYPE
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(DUMP_SEED)
+    R = eng.nsims
+    stat_f = ("ticks", "events", "finished", "started", "placement_evals", "done")
+    win_f = ("ev_rows", "q_rows", "node_events", "spans_used", "admitted")
+    stats = np.zeros((R, 1 + len(stat_f) + len(win_f)))
+    for r in range(R):
+        st, w = eng.stats(r), eng.window(r)
+        stats[r] = [r] + [getattr(st, f) for f in stat_f] + [getattr(w, f) for f in win_f]
+
+    def pick(count, cap):
+        return np.arange(count) if count <= cap else np.sort(rng.choice(count, size=cap, replace=False))
+
+    row_f = [f for f in ROW_DTYPE.names if f != "reserved"]
+    jobs, order, spans, rows = [], [], [], []
+    for r in pick(R, DUMP_REPLICAS):
+        r = int(r)
+        recs, fin = eng.fetch_jobs(r)
+        off, sp = eng.fetch_spans(r)
+        j = pick(len(recs), DUMP_JOBS)
+        jobs.append(np.column_stack([np.full(len(j), r), j] + [recs[f][j] for f in recs.dtype.names]))
+        p = pick(len(fin), DUMP_JOBS)
+        order.append(np.column_stack([np.full(len(p), r), p, fin[p]]))
+        cnt = off[j + 1] - off[j]
+        s = np.repeat(off[j] - (np.cumsum(cnt) - cnt), cnt) + np.arange(cnt.sum())      # the spans of job j[i] in order
+        spans.append(np.column_stack([np.full(len(s), r), np.repeat(j, cnt), sp["node"][s], sp["ntasks"][s], sp["devmask"][s]]))
+        tr = eng.fetch_rows(r, int(eng.window(r).row_first))
+        k = np.union1d(pick(len(tr), DUMP_ROWS - 1), [len(tr) - 1]) if len(tr) else np.zeros(0, dtype=np.int64)
+        rows.append(np.column_stack([np.full(len(k), r)] + [tr[f][k] for f in row_f]))
+    out = {"replica_stats": stats, "jobs": np.concatenate(jobs), "finish_order": np.concatenate(order),
+           "spans": np.concatenate(spans), "rows": np.concatenate(rows)}
+    out = {name: np.ascontiguousarray(a, dtype=np.float64) for name, a in out.items()}
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT}-byte limit")
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    log(f"[dump] {total / 1e6:.1f} MB of outputs -> {out_dir}")
 
 
 def numa_cpus_of_gpu(index):
@@ -342,6 +404,8 @@ def ours(args):
     wall_ms = red.max(wall_ms)
     events_all = red.sum(events_rank)
     value = events_all / (dev_ms / args.steps / 1e3)
+    if args.dump_outputs and rank == 0:                   # rank 0's replicas are those of a one-GPU run
+        dump_outputs(eng, args.dump_outputs)
 
     if args.value_only:
         if rank == 0:
@@ -926,9 +990,11 @@ def horus_mode(args):
     # test harness (tests/emu), one core, same replicas and stream -- what `cpu_tight` is for the fifo engine
     tight = None
     try:
+        import tempfile
         sys.path.insert(0, os.path.join(REPO, "tests"))
         import emu
-        emu.lib()
+        with tempfile.TemporaryDirectory(prefix="gs_emu_") as tmp:
+            emu.lib(os.path.join(tmp, "libhorus_emu.so"))       # loaded: the file may go with the directory
         k = min(R, 256)
         t0 = time.perf_counter()
         tight_ev = sum(emu.run_horus(cluster, hp, tables[r], stream, args.horus_rows)[6] for r in range(k))
@@ -1076,7 +1142,13 @@ def main():
     ap.add_argument("--horus-scalar-only", action="store_true", help="development: time the scalar mapping and stop")
     ap.add_argument("--horus-words", type=int, default=6 << 20, help="raw generator words for the horus+ device check")
     ap.add_argument("--place-jobs", type=int, default=64 * 1024 * 1024)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float64; see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.mode != "sim" or args.impl != "ours" or args.policy != "fifo" or args.only_sharded):
+        ap.error("--dump-outputs writes the outputs of the fifo replica run (the default mode)")
     if args.mode == "place":
         place_mode(args)
     elif args.mode == "horus":

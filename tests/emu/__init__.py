@@ -11,24 +11,26 @@ _OUT = os.path.join(_HERE, "_build", "libhorus_emu.so")
 _lib = None
 
 
-def build(force=False):
+def build(force=False, out=_OUT):
     src = os.path.join(_HERE, "horus_emu.cpp")
     deps = [src, os.path.join(_REPO, "gpuschedule_b200", "csrc", "gs_horus_core.cuh"),
             os.path.join(_REPO, "gpuschedule_b200", "csrc", "gs_horus_host.h"),
             os.path.join(_REPO, "include", "gsched.h"), os.path.join(_REPO, "include", "gsched_horus.h")]
-    if not force and os.path.exists(_OUT) and os.path.getmtime(_OUT) >= max(os.path.getmtime(d) for d in deps):
-        return _OUT
-    os.makedirs(os.path.dirname(_OUT), exist_ok=True)
+    if not force and os.path.exists(out) and os.path.getmtime(out) >= max(os.path.getmtime(d) for d in deps):
+        return out
+    os.makedirs(os.path.dirname(out), exist_ok=True)
     subprocess.run(["g++", "-O2", "-fPIC", "-std=c++17", "-ffp-contract=off", "-shared", "-x", "c++",
                     "-I", os.path.join(_REPO, "include"), "-I", os.path.join(_REPO, "gpuschedule_b200", "csrc"),
-                    "-o", _OUT, src], check=True)
-    return _OUT
+                    "-o", out, src], check=True)
+    return out
 
 
-def lib():
+def lib(out=_OUT):
+    """the host build of the engine's core; `out` is where it is built (bench.py passes a temporary directory,
+    because the tree it runs from may be read-only)"""
     global _lib
     if _lib is None:
-        _lib = C.CDLL(build())
+        _lib = C.CDLL(build(out=out))
         _lib.emu_run_horus.restype = C.c_longlong
     return _lib
 

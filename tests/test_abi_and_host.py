@@ -33,8 +33,9 @@ def test_library_exports_every_declared_symbol():
 
 
 def test_library_is_built_for_sm_100a():
-    from gpuschedule_b200 import capi
-    out = subprocess.run(["cuobjdump", "-lelf", capi.LIB_PATH], capture_output=True, text=True).stdout
+    from gpuschedule_b200 import _build, capi
+    cuobjdump = os.path.join(os.path.dirname(_build.nvcc_path()), "cuobjdump")     # the toolkit need not be on PATH
+    out = subprocess.run([cuobjdump, "-lelf", capi.LIB_PATH], capture_output=True, text=True, check=True).stdout
     assert "sm_100a" in out
 
 
